@@ -4,8 +4,10 @@
 with per-stage achieved HBM GB/s against the measured copy peak, next to the restated
 reference CPU path timed on the same box.
 
-Contract (driver): python bench.py --gpus N --steps K --warmup W [--impl reference]
-  * a "step" = one block of synthetic baseband through the whole chain on each rank;
+Usage: python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
+  * a "step" = one block of synthetic baseband through the whole chain on each rank; every timed window is K steps;
+  * --dump-outputs DIR writes what the last timed step computed (dump_block_outputs) for output-by-output comparison
+    of two builds; apart from that bench.py writes no files (the source tree may be read-only);
   * workload = BASELINE.json configs[2], the J1644-4559 shape the north star names: dual-polarisation
     8-bit, 2^26 samples per stream per block, 400 MHz, DM 562.05, C = 2^11 channels (rows of 2^14 time
     samples), manual zap list, SK and the boxcar detector; one block in two of the ring carries an injected
@@ -50,6 +52,7 @@ os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "8")
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT / "simple-radio-telescope-backend_b200"))
 sys.path.insert(0, str(ROOT / "tests"))
+sys.dont_write_bytecode = True   # no __pycache__ beside the modules imported from the (possibly read-only) tree
 
 import numpy as np  # noqa: E402
 
@@ -592,6 +595,7 @@ class Harness:
         self.detections = 0
         self.blocks_with_detection = 0
         self._tickets = []
+        self.last_block = None
 
     def close(self):
         for c in self.ctxs:
@@ -603,7 +607,8 @@ class Harness:
 
     def _collect(self):
         c, t = self._tickets.pop(0)
-        res = c.collect_block(t)
+        res, h_series, d_spectra = c.collect_block_ex(t)
+        self.last_block = (res, h_series, d_spectra)   # ring-slot buffers: valid until the slot is submitted again
         found = sum(int(r.signal_count[b]) for r in res for b in range(r.n_boxcars))
         self.detections += found
         self.blocks_with_detection += 1 if found else 0
@@ -664,6 +669,52 @@ class Harness:
         return warm
 
 
+DUMP_SPECTRUM_SAMPLES = 1 << 20   # per stream: 8 MiB of the 256 MiB dynamic spectrum of a config3 stream
+DUMP_SEED = 0x53525442
+
+
+class _LibraryDeviceFloats:
+    """a float32 device buffer owned by libsrtb_b200, seen by torch without a copy"""
+
+    def __init__(self, ptr: int, count: int):
+        self.__cuda_array_interface__ = {"shape": (count,), "typestr": "<f4", "data": (ptr, False), "version": 2}
+
+
+def dump_block_outputs(out_dir: str, torch, srtb_b200, H):
+    """Writes what collect_block_ex hands the caller for the last block the timed loop collected, as .npy files:
+    per stream the detector result (entries past n_boxcars zeroed), the boxcar series it marked positive
+    ([stream][boxcar][L], zero elsewhere) and a fixed seeded sample of the dynamic spectrum [C][L] (complex64 as
+    float32 pairs, at the flat indices in spectrum_sample_index). 28 MiB for config3. The blocks are seeded, so the
+    same arguments dump the same outputs from any build."""
+    res, h_series, d_spectra = H.last_block
+    streams, mb = len(res), srtb_b200.MAX_BOXCARS
+    nc = H.n // 2
+    L = nc // min(H.w["channels"], nc)
+    fields = {k: np.zeros((streams, mb), np.float64) for k in ("boxcar_length", "series_length", "signal_count")}
+    fields.update({k: np.zeros((streams, mb), np.float32) for k in ("variance", "threshold")})
+    summary = np.zeros((streams, 4), np.float64)
+    series = np.zeros((streams, mb, L), np.float32)
+    host_series = np.ctypeslib.as_array(C.cast(h_series, C.POINTER(C.c_float)), shape=(streams, mb, L))
+    for s, r in enumerate(res):
+        nb = r.n_boxcars
+        summary[s] = (r.zero_count, r.time_series_count, r.detect_enabled, nb)
+        for k, a in fields.items():
+            a[s, :nb] = getattr(r, k)[:nb]
+        for b in range(nb):
+            if r.signal_count[b] > 0:
+                series[s, b, :r.series_length[b]] = host_series[s, b, :r.series_length[b]]
+    count = min(nc, DUMP_SPECTRUM_SAMPLES)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(nc, count, replace=False))
+    d_idx = torch.from_numpy(idx).cuda()
+    spectrum = np.stack([torch.as_tensor(_LibraryDeviceFloats(d_spectra[s], 2 * nc), device="cuda").view(nc, 2)[d_idx]
+                         .cpu().numpy() for s in range(streams)])
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = dict(detect_summary=summary, series=series, spectrum_sample=spectrum,
+                  spectrum_sample_index=idx.astype(np.float64), **fields)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_dm_sweep(args, torch, srtb_b200, w, wname, rank, local_rank, world, dist):
     """BASELINE config #4: one 2^27-sample block per step, 21 trial DMs each (unpack + R2C once, then s1 + chirp ->
     waterfall -> SK -> detector per DM: srtb_b200_process_block_dm_sweep). Blocks are sharded over the ranks; block 0
@@ -680,7 +731,7 @@ def run_dm_sweep(args, torch, srtb_b200, w, wname, rank, local_rank, world, dist
 
     for i in range(max(args.warmup, 3)):
         step(i, False)
-    steps = max(4, min(args.steps, 40))
+    steps = args.steps
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
@@ -736,7 +787,7 @@ def run_udp_stream(args, torch, w, wname, rank, local_rank, world, dist):
     the unpaced rate the same path sustains."""
     exe = ROOT / "src" / "srtb_b200"
     if not exe.exists():
-        subprocess.run(["make", "-C", str(ROOT / "src")], check=True, capture_output=True)
+        raise SystemExit(f"bench.py: {exe} not built: run __graft_entry__.build() first")
 
     def run(rate, seconds):
         cmd = [str(exe), "--config_file_name", "/nonexistent.cfg", "--gpu_devices", str(local_rank), "--chains_per_gpu", "2",
@@ -811,7 +862,14 @@ def main():
     ap.add_argument("--contexts", type=int, default=int(os.environ.get("SRTB_BENCH_CONTEXTS", "0")),
                     help="contexts per GPU that blocks alternate over (0 = 1 for multi-stream blocks of >= 2^26 samples, whose "
                          "streams the context overlaps itself; else 6 up to 2^24-sample blocks, 4 up to 2^27, 2 above)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0; "
+                         "workloads config1..config3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("config4", "config5")):
+        ap.error("--dump-outputs covers the block-ring path of workloads config1..config3")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     wname = args.workload
     w = WORKLOADS[wname]
@@ -859,6 +917,8 @@ def main():
         sampler.snapshot()          # short run: take one sample while the GPU is still under load
     ms_per_step = ms_total / args.steps
     value = samples_per_step / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_block_outputs(args.dump_outputs, torch, srtb_b200, H)
 
     # ---- end to end from pinned host memory (`e2e`)
     H.warm(H.step_e2e, args.warmup)
@@ -874,7 +934,7 @@ def main():
     if len(H.ctxs) > 1:
         extra, H.ctxs, H.extra_streams = (H.ctxs[1:], H.extra_streams), H.ctxs[:1], []
         H.warm(H.step_device, args.warmup)
-        ms1 = H.timed(H.step_device, max(10, args.steps // 2), dist) / max(10, args.steps // 2)
+        ms1 = H.timed(H.step_device, args.steps, dist) / args.steps
         single = {"value": samples_per_step / (ms1 * 1e-3) / 1e9, "unit": UNIT, "ms_per_step": ms1, "contexts_per_gpu": 1}
         H.ctxs, H.extra_streams = H.ctxs + extra[0], extra[1]
     else:
@@ -1004,7 +1064,7 @@ def main():
         torch.cuda.empty_cache()
         w2 = WORKLOADS[args.secondary]
         H2 = Harness(torch, srtb_b200, args.secondary, w2, default_contexts(w2), rank, local_rank, inject_pulse=False)
-        steps2 = max(args.steps, 200)
+        steps2 = args.steps
         H2.warm(H2.step_device, args.warmup)
         ms2 = H2.timed(H2.step_device, steps2, dist) / steps2
         H2.warm(H2.step_e2e, args.warmup)

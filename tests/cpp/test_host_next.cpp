@@ -91,7 +91,7 @@ int main(int argc, char** argv) {
   CHECK(c.udp_receiver_address.size() == 2 && c.udp_receiver_address[1] == "10.0.1.3");
   CHECK(srtb::log::current_level == srtb::log::levels::DEBUG);
   srtb::log::current_level = srtb::log::levels::WARNING;
-  // the two shipped configuration files, verbatim, when the reference tree is present (argv[2] = its userspace dir):
+  // the reference's two example configuration files, verbatim (argv[2] = the directory holding them, tests/golden):
   // srtb_config.cfg:2-22 and srtb_config_1644-4559.cfg:2-29 must load into srtb::configs unchanged
   if (argc > 2) {
     const std::string ref = argv[2];

@@ -34,6 +34,36 @@ def test_gpu_arm_fails_loudly_without_a_device():
     assert "no CUDA device" in r.stderr or "no CPU fallback" in r.stderr
 
 
+def test_bad_arguments_are_refused_before_any_work():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"],
+                  ["--workload", "config5", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--warmup", "0", *extra],
+                           capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and r.stdout.strip() == "" and "error:" in r.stderr, extra
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_reproducible(tmp_path):
+    """--dump-outputs: two runs with the same arguments write the same arrays (float32 / float64, <= 64 MiB)"""
+    import numpy as np
+    dumps = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "0",
+                            "--workload", "config2", "--secondary", "none", "--no-cpu-baseline", "--stage-iters", "1",
+                            "--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-1500:]
+        assert json.loads(r.stdout)["steps"] == 3
+        dumps.append({p.stem: np.load(p) for p in sorted((tmp_path / run).glob("*.npy"))})
+    a, b = dumps
+    assert {"detect_summary", "signal_count", "series", "spectrum_sample", "spectrum_sample_index"} <= set(a)
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert a["detect_summary"].shape == (1, 4) and a["detect_summary"][0, 2] == 1      # one stream, detector enabled
+    assert np.abs(a["spectrum_sample"]).sum() > 0
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+
+
 def test_both_arms_name_the_same_workload_and_default_is_the_j1644_shape():
     """the driver compares config.workload of the two arms; the default is BASELINE configs[2] (north star)"""
     sys.path.insert(0, str(ROOT))
